@@ -26,6 +26,12 @@ configs[1], weak scaling: frames shard by batch, no data-path collective), whole
   c4 / c5   : BASELINE configs[3] / [4] (multi-camera pipeline; YOLOv9-e + CLIP all-gather), emitted when N > 1 or on
               request
 
+--dump-outputs DIR: after the timed steps, what the detector's and CLIP's timed paths returned in their last step, as
+DIR/<name>.npy (float32; `.rank<r>` before `.npy` when N > 1): detections and e2e_detections (B,300,6), the detector head
+of the last step's first two frames (2,84,anchors), and per CLIP tower <arch>_image_embeddings, <arch>_crop_embeddings and
+<arch>_text_embeddings (256, embed_dim).  Weights and inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
+
 oracle/ is imported here for three things only: the CPU legs, a small parity sample printed with the CPU leg, and — before
 any timed region — the seeded synthetic weights and frames every arm runs on.  Every timed GPU region calls clearcam_b200
 alone.
@@ -235,10 +241,9 @@ def cpu_pool(task, P, steps, warmup=2):
         layout = f"{nproc} pinned worker processes x {threads} torch threads"
         units = nproc * steps * upc
         if nproc > 1:
-            solo_steps = max(2, steps // 2)
-            r1, w1 = _cpu_pool_run(task, d, 1, threads, solo_steps, warmup, pin=False)
+            r1, w1 = _cpu_pool_run(task, d, 1, threads, steps, warmup, pin=False)
             if r1 > rate:
-                rate, wall, units = r1, w1, solo_steps * upc
+                rate, wall, units = r1, w1, steps * upc
                 layout = f"1 worker process x {threads} torch threads (faster than {nproc} workers x {threads} threads on this box)"
                 nproc = 1
     return {"value": rate, "unit": CPU_TASKS[task]["unit"], "cores": nproc * threads, "kind": "port",
@@ -249,11 +254,11 @@ def cpu_pool(task, P, steps, warmup=2):
 
 def run_reference(args):
     """--impl reference: the reference's own CPU implementation of the path, restated (oracle/): tinygrad DEV=CPU cannot
-    run here.  A step = every worker runs one oracle call (4 frames / 8 crops); `--steps` is honoured up to 40."""
+    run here.  A step = every worker runs one oracle call (4 frames / 8 crops)."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
     clip = args.workload == "clip"
-    steps = max(1, min(args.steps, 40))
+    steps = args.steps
     warm = max(1, min(args.warmup, 3))
     if clip:
         from oracle import clip as oc
@@ -329,6 +334,17 @@ class Ctx:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return float(t.item())
 
+    def dump(self, **arrays):
+        """--dump-outputs: write each tensor as DIR/<name>.npy in float32."""
+        d = self.args.dump_outputs
+        if not d:
+            return
+        import numpy as np
+        os.makedirs(d, exist_ok=True)
+        sfx = f".rank{self.rank}" if self.world > 1 else ""
+        for name, t in arrays.items():
+            np.save(os.path.join(d, f"{name}{sfx}.npy"), t.detach().to("cpu", torch.float32).numpy())
+
 
 def yolo_section(cx, with_cpu):
     from oracle import yolov9 as o
@@ -356,7 +372,11 @@ def yolo_section(cx, with_cpu):
     sampler = ClockSampler(cx.local)
     if rank == 0:
         sampler.start()
-    ms_total = cx.timed(lambda i: model.detect_batch(dev_batches[i % nbuf]), K)
+    last = {}
+
+    def step(i):
+        last["detections"] = model.detect_batch(dev_batches[i % nbuf])
+    ms_total = cx.timed(step, K)
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * K / (ms_total / 1000.0)
 
@@ -368,9 +388,17 @@ def yolo_section(cx, with_cpu):
     def e2e_all(_):
         for r in model.detect_pipelined(host_batches[i % 2] for i in range(K)):
             n_out[0] += r.shape[0]
+            last["e2e_detections"] = r
     ms_e2e = cx.timed(e2e_all, 1)
     assert n_out[0] == B * K
     e2e = world * B * K / (ms_e2e / 1000.0)
+    if args.dump_outputs:
+        # these synthetic frames give few or no boxes above the 0.25 threshold (none in the last step at the defaults), so the
+        # detections alone say little: add the head tensor they are selected from (boxes, class probabilities) for the last
+        # step's input, frames 0 and 1
+        _, raw = model.detect_batch(dev_batches[(K - 1) % nbuf], raw=True)
+        last["head"] = raw[:2]
+    cx.dump(**last)
 
     line = None
     if rank == 0:
@@ -475,10 +503,14 @@ def clip_section(cx, with_cpu, archs=(("ViT-B/32", 256), ("ViT-L/14", 256))):
         xs = [oc.synthetic_images(8, cfg.image_size, seed=10 + i)[torch.arange(cb) % 8].cuda() for i in range(3)]
         for i in range(3):
             cm.precompute_embedding(xs[i % 3], gather=world > 1)
-        steps_c = max(3, min(K, 10))
-        ms = cx.timed(lambda i: cm.precompute_embedding(xs[i % 3], gather=world > 1), steps_c)
-        ips = world * cb * steps_c / (ms / 1000.0)
-        r = {"batch_per_gpu": cb, "value": ips, "unit": "images/s", "ms_per_step": ms / steps_c,
+        tag = arch.replace("ViT-", "vit_").replace("/", "").lower()          # ViT-B/32 -> vit_b32
+        last = {}
+
+        def image_step(i):
+            last[f"{tag}_image_embeddings"] = cm.precompute_embedding(xs[i % 3], gather=world > 1).tensor
+        ms = cx.timed(image_step, K)
+        ips = world * cb * K / (ms / 1000.0)
+        r = {"batch_per_gpu": cb, "value": ips, "unit": "images/s", "ms_per_step": ms / K,
              "tflops": ips * oc.flops_image(cfg) / 1e12, "gflop_per_image": oc.flops_image(cfg) / 1e9, "all_gather": world > 1}
         # e2e: 16 pinned host 720p frames, 16 object rectangles each (= cb crops) -> embeddings on the host
         nfr = 16
@@ -499,8 +531,9 @@ def clip_section(cx, with_cpu, archs=(("ViT-B/32", 256), ("ViT-L/14", 256))):
             torch.cuda.current_stream().synchronize()
         for _ in range(2):
             e2e_step(0)
-        ms = cx.timed(e2e_step, steps_c)
-        r["e2e"] = {"value": world * cb * steps_c / (ms / 1000.0), "unit": "images/s", "h2d_bytes_per_step": hf.numel(),
+        ms = cx.timed(e2e_step, K)
+        last[f"{tag}_crop_embeddings"] = hout
+        r["e2e"] = {"value": world * cb * K / (ms / 1000.0), "unit": "images/s", "h2d_bytes_per_step": hf.numel(),
                     "d2h_bytes_per_step": hout.numel() * 4,
                     "how": f"{nfr} pinned 720p uint8 frames + {cb} rectangles -> ObjectFinder.embed_crops -> pinned host embeddings, synchronous per step"}
         # text tower
@@ -509,9 +542,13 @@ def clip_section(cx, with_cpu, archs=(("ViT-B/32", 256), ("ViT-L/14", 256))):
         ids = oc.pad_tokens([torch.randint(1000, 40000, (int(n),), generator=g).tolist() for n in torch.randint(3, 20, (qb,), generator=g)]).int().cuda()
         for _ in range(2):
             cm.encode_token_ids(ids)
-        ms = cx.timed(lambda i: cm.encode_token_ids(ids), steps_c)
-        r["text"] = {"batch_per_gpu": qb, "queries_per_s": world * qb * steps_c / (ms / 1000.0),
-                     "tflops": world * qb * steps_c / (ms / 1000.0) * oc.flops_text(cfg) / 1e12}
+
+        def text_step(i):
+            last[f"{tag}_text_embeddings"] = cm.encode_token_ids(ids).tensor
+        ms = cx.timed(text_step, K)
+        cx.dump(**last)
+        r["text"] = {"batch_per_gpu": qb, "queries_per_s": world * qb * K / (ms / 1000.0),
+                     "tflops": world * qb * K / (ms / 1000.0) * oc.flops_text(cfg) / 1e12}
         if rank == 0:
             cm._encode_text("a person walking a dog", realize=True)
             torch.cuda.synchronize()
@@ -593,7 +630,7 @@ def c4_section(cx):
     for t in range(3):
         step(t)
     counts["frames"] = counts["crops"] = 0
-    K = max(5, min(cx.args.steps, 20))
+    K = cx.args.steps
     ms = cx.timed(step, K)
     tot = torch.tensor([counts["frames"], counts["crops"]], device="cuda", dtype=torch.float64)
     if world > 1:
@@ -634,7 +671,7 @@ def c5_section(cx):
             cx.dist.all_gather_into_tensor(full, full[rank * 2 * B:(rank + 1) * 2 * B])
     for i in range(3):
         step(i)
-    K = max(5, min(cx.args.steps, 20))
+    K = cx.args.steps
     ms = cx.timed(step, K)
     fps = world * B * K / (ms / 1000.0)
     out = {"workload": f"YOLOv9-e, {B} uint8 640x640 frames per GPU per step ({world * B} in total) + ViT-B/32 embeddings of {2 * B} crops per GPU + all-gather",
@@ -661,7 +698,13 @@ def main():
     ap.add_argument("--sync-dir", default="", help=argparse.SUPPRESS)
     ap.add_argument("--worker-id", type=int, default=0, help=argparse.SUPPRESS)
     ap.add_argument("--pin", default="", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs of the detector and CLIP paths as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("c4", "c5")):
+        ap.error("--dump-outputs covers the detector and CLIP paths: workloads yolo and clip, not --impl reference")
     if args.cpu_worker:
         return cpu_worker(args)
     if args.impl == "reference":
@@ -691,13 +734,13 @@ def main():
         if cx.rank == 0:
             b = r["ViT-B/32"]
             line = {"metric": "images/s CLIP ViT-B/32 224px", "value": b["value"], "unit": "images/s", "n_gpus": cx.world,
-                    "steps": max(3, min(args.steps, 10)), "warmup": 3, "ms_per_step": b["ms_per_step"], "higher_is_better": True,
+                    "steps": args.steps, "warmup": 3, "ms_per_step": b["ms_per_step"], "higher_is_better": True,
                     "scaling": "weak", "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
                     "config": {"workload": CLIP_WORKLOAD, "global_batch": cx.world * 256, "weights": "seeded synthetic",
                                "l2": "3 rotating input batches of 154 MB (> 126 MB L2)",
                                "parallelism": f"dp{cx.world} (crops sharded by batch; in-place all-gather of the embeddings when N > 1)"},
                     "e2e": b["e2e"], "roofline": b.get("roofline"), "cpu_baseline": b.get("cpu_baseline"), "text": b["text"],
-                    "gpu_launches": b.get("launches_per_step", 0) * max(3, min(args.steps, 10)), "ViT-L/14": r["ViT-L/14"]}
+                    "gpu_launches": b.get("launches_per_step", 0) * args.steps, "ViT-L/14": r["ViT-L/14"]}
     else:
         r = (c4_section if args.workload == "c4" else c5_section)(cx)
         if cx.rank == 0:

@@ -4,6 +4,7 @@
   yolov9t_mot16.npz: real YOLOv9-t weights + one real frame + the reference's recorded detections (see below)
   clip_tokens.json : token ids of fixed prompts from the reference's own utils/clip_tokenizer.py (imported, not copied)
                      -> pins clearcam_b200/utils/clip_tokenizer.py (tests/test_tokenizer_cpu.py)
+  clip_tokens_random.json: the same for 300 generated texts (tests/test_oracle_cpu.py)
 """
 import json
 import os
@@ -31,6 +32,24 @@ def main():
         json.dump(out, f, ensure_ascii=True, indent=0)
     print("wrote clip_tokens.json:", len(PROMPTS), "prompts")
 
+
+WORDS = ["person", "Ferrari", "F40", "don't", "it's", "we'll", "I'M", "dog's", "naïve", "café", "Zürich", "北京", "мотоцикл", "🚗", "😀",
+         "&amp;", "&lt;b&gt;", "3.14", "1080p", "a", "THE", "x-ray", "e-mail", "#tag", "@home", "100%", "(red)", "white/blue", "...",
+         "  ", "\t", "van", "ladder", "night-time", "ＦＵＬＬ", "ﬁre", "o'clock", "10:30", "$5", "état", "straße"]
+
+
+def make_random_tokens():
+    """clip_tokens_random.json: 300 generated texts (mixed case, digits, punctuation, apostrophe forms, runs of spaces,
+    accented and non-Latin characters, emoji, html entities) and the reference tokenizer's ids for them."""
+    import numpy as np
+    sys.path.insert(0, REF)
+    from utils.clip_tokenizer import SimpleTokenizer
+    tok = SimpleTokenizer()
+    rng = np.random.default_rng(0)
+    texts = [" ".join(WORDS[int(i)] for i in rng.integers(0, len(WORDS), int(rng.integers(1, 9)))) for _ in range(300)]
+    out = {"source": "reference utils/clip_tokenizer.py SimpleTokenizer.encode", "texts": texts, "ids": [tok.encode(t) for t in texts]}
+    with open(os.path.join(ROOT, "tests", "golden", "clip_tokens_random.json"), "w") as f:
+        json.dump(out, f, ensure_ascii=True, separators=(",", ":"))
 
 
 
@@ -62,4 +81,5 @@ def make_yolov9t_fixture():
 
 if __name__ == "__main__":
     main()
+    make_random_tokens()
     make_yolov9t_fixture()

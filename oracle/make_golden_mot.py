@@ -13,8 +13,9 @@ Measured here: 156 people tracks = the reference's known answer.  The statistic 
 chain gives 159 with the channel swap, 155 with the bf16-mirror oracle and 153 from the older-revision detections stored
 in test/tracks.pkl.
 
-    python oracle/make_golden_mot.py        # ~100 s on 8 cores
+    CLEARCAM_B200_MOT_VIDEO=<the reference's test/videos/MOT16-03.mp4> python oracle/make_golden_mot.py    # ~100 s on 8 cores
 """
+import os
 import sys
 from pathlib import Path
 
@@ -23,6 +24,7 @@ import torch
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
+VIDEO = os.environ.get("CLEARCAM_B200_MOT_VIDEO", "")
 
 
 def count_people(dets, tracker):
@@ -41,7 +43,7 @@ def main():
     from oracle import yolov9 as o
     g = np.load(ROOT / "tests" / "golden" / "yolov9t_mot16.npz")
     P = {k[2:]: torch.from_numpy(g[k]) for k in g.keys() if k.startswith("w:")}
-    cap = cv2.VideoCapture("/root/reference/test/videos/MOT16-03.mp4")
+    cap = cv2.VideoCapture(VIDEO)
     dets = []
     while True:
         ret, im = cap.read()
@@ -57,5 +59,21 @@ def main():
     np.savez_compressed(ROOT / "tests" / "golden" / "mot16_oracle_dets.npz", dets=dets, people=n_ref, expected=156)
 
 
+def make_frame1():
+    """mot16_frame1.npz: frame 1 of the video as its difference from frame 0 (the frame stored in yolov9t_mot16.npz); the
+    camera is static, so the difference compresses to a few KB.  tests/test_oracle_cpu.py runs the oracle on frames 0 and 1
+    and compares with the stored detections."""
+    import cv2
+    f0 = np.load(ROOT / "tests" / "golden" / "yolov9t_mot16.npz")["frame"]
+    cap = cv2.VideoCapture(VIDEO)
+    ok0, im0 = cap.read()
+    ok1, im1 = cap.read()
+    assert ok0 and ok1 and np.array_equal(im0, f0)
+    d = im1.astype(np.int16) - f0
+    assert np.abs(d).max() < 128
+    np.savez_compressed(ROOT / "tests" / "golden" / "mot16_frame1.npz", delta_from_frame0=d.astype(np.int8))
+
+
 if __name__ == "__main__":
     main()
+    make_frame1()

@@ -11,8 +11,12 @@ from /root/reference — only possible in the build container) and stores inputs
                                     and with the BYTE stage on
   tests/golden/ocsort_synth.npz     three seeded synthetic scenes (crossing boxes, drop-outs, low-score rows, class flips)
                                     through the reference with other constructor arguments (use_byte, max_age, delta_t)
+  tests/golden/ocsort_random.npz    twelve shorter seeded scenes, each with randomly drawn constructor arguments, through
+                                    the reference; only the outputs are stored, the test regenerates the frames from the
+                                    seeds with synthetic_scene()
 
-Per frame the stored output rows are [tl_x, tl_y, w, h, score, class_id, track_id, tracklet_len, speed] (float64).
+Per frame the stored output rows are [tl_x, tl_y, w, h, score, class_id, track_id, tracklet_len, speed] (float64; float32
+in ocsort_random.npz).
 
     python oracle/make_golden_ocsort.py
 """
@@ -81,6 +85,29 @@ def synthetic_scene(seed, n_frames=240, n_obj=14, W=1280, H=720):
     return np.stack(frames)
 
 
+RANDOM_SEEDS = range(100, 112)
+
+
+def random_scene(seed):
+    """(frames, det_thresh, OCSort kwargs) of the random scene `seed`: constructor arguments, threshold and object count
+    are drawn from the seed too."""
+    g = np.random.default_rng(seed)
+    kw = dict(max_age=int(g.choice([5, 30, 100])), min_hits=int(g.choice([1, 3])), iou_threshold=float(g.choice([0.2, 0.3, 0.5])),
+              delta_t=int(g.choice([1, 2, 3])), inertia=float(g.choice([0.0, 0.2, 0.4])), use_byte=bool(g.integers(0, 2)))
+    thr = float(g.choice([0.25, 0.4, 0.5]))
+    return synthetic_scene(seed, n_frames=100, n_obj=int(g.integers(3, 25))), thr, kw
+
+
+def make_random_scenes():
+    out = {}
+    for seed in RANDOM_SEEDS:
+        frames, thr, kw = random_scene(seed)
+        rows, offs = run_reference(frames, thr, **kw)
+        out[f"{seed}_rows"], out[f"{seed}_offsets"] = rows.astype(np.float32), offs.astype(np.int32)     # float32: far below rtol 1e-5
+        out[f"{seed}_frames_sum"] = frames.astype(np.float64).sum()      # detects a change of synthetic_scene's output
+    np.savez_compressed(OUT / "ocsort_random.npz", **out)
+
+
 def main():
     OUT.mkdir(parents=True, exist_ok=True)
     sys.path.insert(0, str(REF))
@@ -117,6 +144,7 @@ def main():
         out[f"{name}_args"] = np.array([thr, kw["max_age"], float(kw.get("use_byte", False))])
         print("tracker_inputs", name, rows.shape, "ids up to", rows[:, 6].max())
     np.savez_compressed(OUT / "ocsort_street.npz", **out)
+    make_random_scenes()
 
 
 if __name__ == "__main__":

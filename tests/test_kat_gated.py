@@ -3,7 +3,7 @@
   * CLIP: the reference's real ViT-L/14 weights (models/objects.py:91 downloads CLIP-ViT-L-14-laion2B-s32B-b82K.safetensors)
     under $CLEARCAM_B200_WEIGHTS -> test/test_clip.py's 0.330654 and the embeddings stored in test/clip_images/embeddings.pkl
     (fixtures: tests/golden/clip_kat.npz from oracle/make_golden_clip_kat.py), for the CPU oracle and for the CUDA path.
-  * Detector + tracker: the reference's test/videos/MOT16-03.mp4 (11 MB) at $CLEARCAM_B200_MOT_VIDEO (or in /root/reference)
+  * Detector + tracker: the reference's test/videos/MOT16-03.mp4 (11 MB) at $CLEARCAM_B200_MOT_VIDEO
     -> test/run_mot.py's 156 distinct moving person tracks through the CUDA detector (YOLOv9-t weights recovered from the
     reference's iOS bundle, tests/golden/yolov9t_mot16.npz) and the C++ tracker.
 Until then CLIP numerics stay "parity unpinned" (DESIGN.md §2)."""
@@ -17,10 +17,9 @@ import torch
 GOLD = Path(__file__).parent / "golden"
 W_NAME = "CLIP-ViT-L-14-laion2B-s32B-b82K.safetensors"
 W_PATH = Path(os.environ.get("CLEARCAM_B200_WEIGHTS", "/nonexistent")) / W_NAME
-VIDEO = next((p for p in (os.environ.get("CLEARCAM_B200_MOT_VIDEO", ""), str(Path(__file__).parent.parent / "tmp_mot16.mp4"),
-                          "/root/reference/test/videos/MOT16-03.mp4") if p and os.path.exists(p)), None)
+VIDEO = os.environ.get("CLEARCAM_B200_MOT_VIDEO", "")
 needs_clip_weights = pytest.mark.skipif(not W_PATH.exists(), reason=f"real CLIP weights not found at {W_PATH}")
-needs_video = pytest.mark.skipif(VIDEO is None, reason="MOT16-03.mp4 not available (set $CLEARCAM_B200_MOT_VIDEO)")
+needs_video = pytest.mark.skipif(not os.path.isfile(VIDEO), reason="MOT16-03.mp4 not available (set $CLEARCAM_B200_MOT_VIDEO)")
 
 
 def _kat():

@@ -116,28 +116,24 @@ def test_contract_edges():
 
 
 def test_live_against_the_reference_tracker_on_random_scenes():
-    """Where the reference checkout is present (the build container; never on the GPU box), run ITS tracker side by side on
-    fresh random scenes and constructor arguments.  Everything must agree frame by frame except the *numbering* of tracks
-    born in the same frame: that order comes from how the reference's np.argsort happens to order exactly equal costs
-    (zero-cost pairs of non-overlapping boxes), which numpy leaves unspecified and which differs between CPUs (SIMD sort
-    dispatch).  So ids are compared up to one consistent relabelling per scene, rows as sets."""
-    import os
+    """Twelve seeded random scenes with randomly drawn constructor arguments against the reference tracker's output on them
+    (ocsort_random.npz, from oracle/make_golden_ocsort.py; the frames are regenerated here from the seeds).  Everything must
+    agree frame by frame except the *numbering* of tracks born in the same frame: that order comes from how the reference's
+    np.argsort happens to order exactly equal costs (zero-cost pairs of non-overlapping boxes), which numpy leaves unspecified
+    and which differs between CPUs (SIMD sort dispatch).  So ids are compared up to one consistent relabelling per scene,
+    rows as sets."""
     import sys
-    if not os.path.isdir("/root/reference/ocsort_tracker"):
-        pytest.skip("reference checkout not available")
     sys.path.insert(0, str(Path(__file__).parent.parent / "oracle"))
     import warnings
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        from make_golden_ocsort import run_reference, synthetic_scene
+        from make_golden_ocsort import RANDOM_SEEDS, random_scene
+        gold = np.load(GOLD / "ocsort_random.npz")
         relabelled = 0
-        for seed in range(100, 112):
-            g = np.random.default_rng(seed)
-            kw = dict(max_age=int(g.choice([5, 30, 100])), min_hits=int(g.choice([1, 3])), iou_threshold=float(g.choice([0.2, 0.3, 0.5])),
-                      delta_t=int(g.choice([1, 2, 3])), inertia=float(g.choice([0.0, 0.2, 0.4])), use_byte=bool(g.integers(0, 2)))
-            thr = float(g.choice([0.25, 0.4, 0.5]))
-            frames = synthetic_scene(seed, n_frames=100, n_obj=int(g.integers(3, 25)))
-            rows, offs = run_reference(frames, thr, **kw)
+        for seed in RANDOM_SEEDS:
+            frames, thr, kw = random_scene(seed)
+            assert frames.astype(np.float64).sum() == gold[f"{seed}_frames_sum"], f"seed {seed}: synthetic_scene changed"
+            rows, offs = gold[f"{seed}_rows"].astype(np.float64), gold[f"{seed}_offsets"]
             trk, ids = ocsort.OCSort(**kw), {}
             for i in range(len(frames)):
                 got = _as_rows(trk.update(frames[i], thr))

@@ -212,29 +212,15 @@ def test_zero_padded_equivalent_computes_the_same_function(size):
 
 
 def test_tokenizer_live_against_the_reference_on_random_text():
-    """Build container only: the reference's own tokenizer module (pure Python) side by side on generated text — mixed case,
-    digits, punctuation, apostrophe forms, runs of spaces, accented and non-Latin characters, emoji, html entities."""
-    import importlib.util
-    ref_py = "/root/reference/utils/clip_tokenizer.py"
-    if not os.path.exists(ref_py):
-        pytest.skip("reference checkout not available")
-    spec = importlib.util.spec_from_file_location("_ref_clip_tokenizer", ref_py)
-    ref = importlib.util.module_from_spec(spec)
-    try:
-        spec.loader.exec_module(ref)
-        rt = ref.SimpleTokenizer()
-    except Exception as ex:                                   # the reference module wants ftfy/regex: skip if it cannot load here
-        pytest.skip(f"reference tokenizer not importable here: {ex!r}")
+    """300 generated texts — mixed case, digits, punctuation, apostrophe forms, runs of spaces, accented and non-Latin
+    characters, emoji, html entities — against the ids the reference's own tokenizer module gave for them
+    (clip_tokens_random.json, from oracle/make_golden.py)."""
     from clearcam_b200.utils.clip_tokenizer import SimpleTokenizer
     tok = SimpleTokenizer()
-    rng = np.random.default_rng(0)
-    words = ["person", "Ferrari", "F40", "don't", "it's", "we'll", "I'M", "dog's", "naïve", "café", "Zürich", "北京", "мотоцикл", "🚗", "😀",
-             "&amp;", "&lt;b&gt;", "3.14", "1080p", "a", "THE", "x-ray", "e-mail", "#tag", "@home", "100%", "(red)", "white/blue", "...",
-             "  ", "\t", "van", "ladder", "night-time", "ＦＵＬＬ", "ﬁre", "o'clock", "10:30", "$5", "état", "straße"]
-    for _ in range(300):
-        n = int(rng.integers(1, 9))
-        text = " ".join(words[int(i)] for i in rng.integers(0, len(words), n))
-        assert tok.encode(text) == rt.encode(text), repr(text)
+    gold = json.load(open(os.path.join(GOLD, "clip_tokens_random.json")))
+    assert len(gold["texts"]) == 300
+    for text, ids in zip(gold["texts"], gold["ids"]):
+        assert tok.encode(text) == ids, repr(text)
 
 
 def test_reference_known_answer_156_people_tracks_on_mot16():
@@ -254,18 +240,14 @@ def test_reference_known_answer_156_people_tracks_on_mot16():
             if x.class_id == 0:
                 ppl.add(x.track_id)
     assert len(ppl) == 156
-    # tie the stored detections to the oracle code where the reference's video can be read (build container only)
-    video = "/root/reference/test/videos/MOT16-03.mp4"
-    if os.path.exists(video):
-        cv2 = pytest.importorskip("cv2")
-        w = np.load(os.path.join(GOLD, "yolov9t_mot16.npz"))
-        P = {k[2:]: torch.from_numpy(w[k]) for k in w.keys() if k.startswith("w:")}
-        cap = cv2.VideoCapture(video)
-        for i in range(2):
-            ok, im = cap.read()
-            assert ok
-            with torch.no_grad():
-                pred = o.detect("t", P, torch.from_numpy(im).float()[None], 960, bgr_swap=False)[0].numpy()
-            live = dets[i][:, 4] > 0
-            assert (pred[:, 4] > 0).sum() == live.sum()
-            np.testing.assert_allclose(pred[live], dets[i][live], rtol=0, atol=2e-2)
+    # tie the stored detections to the oracle code: its detections on the video's first two frames
+    w = np.load(os.path.join(GOLD, "yolov9t_mot16.npz"))
+    P = {k[2:]: torch.from_numpy(w[k]) for k in w.keys() if k.startswith("w:")}
+    f0 = w["frame"]
+    f1 = (f0 + np.load(os.path.join(GOLD, "mot16_frame1.npz"))["delta_from_frame0"]).astype(np.uint8)
+    for i, im in enumerate((f0, f1)):
+        with torch.no_grad():
+            pred = o.detect("t", P, torch.from_numpy(im).float()[None], 960, bgr_swap=False)[0].numpy()
+        live = dets[i][:, 4] > 0
+        assert (pred[:, 4] > 0).sum() == live.sum()
+        np.testing.assert_allclose(pred[live], dets[i][live], rtol=0, atol=2e-2)
